@@ -27,6 +27,8 @@ GPUs run N x 64 devices (scaling = "weak").
            bounded sample of the workload: one pinned thread per device (multiple_demod_threads mode) and the reference's
            default single-thread round-robin, plus the cfg1 point.
 `--impl reference` times that CPU path alone (rank 0 only under torchrun) and prints the same line shape.
+`--dump-outputs DIR` writes what the e2e leg's caller received in its last timed step (see dump_outputs); the inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -217,6 +219,27 @@ def measured_peaks():
     return {"hbm_gbs": 6650.0}, "fallback"
 
 
+DUMP_BYTES = 48 << 20  # --dump-outputs: above this, a fixed seeded sample of the channels is written
+
+
+def dump_outputs(dirname: str, runs) -> dict:
+    """Write the engine runs of one step, runs = [(waveout[dev][NB_RUN, C, B], axcindicate[dev][NB_RUN, C]), ...] in time
+    order, as dirname/waveout.npy float32 [batches, channels, B] and dirname/axcindicate.npy float32 [batches, channels]
+    (the status characters' codes).  Channels are numbered across devices; all of them when they fit DUMP_BYTES, else a
+    sample drawn with seed 0."""
+    G, B = sum(w.shape[1] for w in runs[0][0]), runs[0][0][0].shape[2]
+    nb = len(runs) * NB_RUN
+    k = min(G, max(1, DUMP_BYTES // (nb * B * 4)))
+    sel = np.arange(G) if k == G else np.sort(np.random.default_rng(0).choice(G, k, replace=False))
+    wave = np.concatenate([np.concatenate(w, axis=1)[:, sel] for (w, _) in runs], axis=0)
+    axc = np.concatenate([np.concatenate(a, axis=1)[:, sel] for (_, a) in runs], axis=0).astype(np.float32)
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "waveout.npy"), wave)
+    np.save(os.path.join(dirname, "axcindicate.npy"), axc)
+    return {"dir": dirname, "waveout": list(wave.shape), "axcindicate": list(axc.shape),
+            "channels": "all" if k == G else f"{k} of {G}, drawn with numpy default_rng(0)"}
+
+
 def source_sha(*rel_paths) -> str:
     h = hashlib.sha256()
     for rp in rel_paths:
@@ -402,8 +425,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the legs of the other BASELINE configs")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle parity spots of the legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the audio and squelch flags the e2e leg fetched in its last timed step "
+                                                          "as DIR/*.npy (rank 0)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.no_e2e):
+        raise SystemExit("--dump-outputs writes what the B200 arm's e2e leg computed: it cannot go with --impl reference or --no-e2e")
     if args.batches_per_step % NB_RUN:
         raise SystemExit(f"--batches-per-step must be a multiple of {NB_RUN}")
     runs_per_step = args.batches_per_step // NB_RUN
@@ -569,8 +598,12 @@ def main():
         step_items = [NB_RUN * B * hop[d] * 2 for d in range(D)]          # array items per engine run per device
         prime_items = [(100 * hop[d] + cfg.fft_size) * 2 for d in range(D)]
         pinned = [torch.from_numpy(np.ascontiguousarray(raws[d][:prime_items[d] + step_items[d]])).pin_memory() for d in range(D)]
-        wo = [np.empty((NB_RUN, len(cfg.devices[d].channels), B), np.float32) for d in range(D)]
-        ax = [np.empty((NB_RUN, len(cfg.devices[d].channels)), np.uint8) for d in range(D)]
+        # the caller's arrays; with --dump-outputs every run of a step fetches into its own (written here, so that no page is
+        # first touched inside the timed loop)
+        keep = runs_per_step if args.dump_outputs else 1
+        wo = [[np.full((NB_RUN, len(cfg.devices[d].channels), B), 0, np.float32) for d in range(D)] for _ in range(keep)]
+        ax = [[np.full((NB_RUN, len(cfg.devices[d].channels)), 0, np.uint8) for d in range(D)] for _ in range(keep)]
+        collected = [0]
         item = [cfg.devices[d].bytes_per_sample for d in range(D)]
 
         def submit(first: bool):
@@ -584,8 +617,10 @@ def main():
             assert n == D * NB_RUN, (n, D * NB_RUN)
 
         def collect():
+            k = collected[0] % keep
             for d in range(D):
-                assert eng2.fetch_many_into(d, NB_RUN, wo[d], ax[d]) == NB_RUN
+                assert eng2.fetch_many_into(d, NB_RUN, wo[k][d], ax[k][d]) == NB_RUN
+            collected[0] += 1
 
         submit(True)
         for _ in range(max(args.warmup, 1) * min(runs_per_step, 4)):
@@ -609,6 +644,9 @@ def main():
                "pcie": pcie, "pcie_frac": (h2d_step * args.steps / dt / 1e9) / pcie["h2d_gbs"] if pcie else None, "numa": numa}
         if pcie and e2e["pcie_frac"] > 1.0:
             e2e["pcie_note"] = "the streaming path moved bytes faster than the copy-rate probe: the probe understates this box's H2D rate"
+        if args.dump_outputs and rank == 0:
+            last = [(collected[0] - keep + i) % keep for i in range(keep)]  # the step's runs, oldest first
+            e2e["dump_outputs"] = dump_outputs(args.dump_outputs, [(wo[k], ax[k]) for k in last])
         eng2.close()
         del pinned
 

@@ -55,6 +55,8 @@ struct pattern_dev_data_t {
     long repeat;                 // the block is sent this many times, then the input reports INPUT_FAILED (end of stream)
     double speedup;              // > 0: paced by the wall clock at speedup x sample_rate, never waits (a full ring
                                  // overflows, input-helpers.cpp:56-60); 0: as fast as the ring drains, lossless
+    size_t written;              // end of the stream bytes appended so far, stored before each append: stream byte s sits in
+                                 // ring slot s % buf_size, so a reader of byte s knows it intact while written <= s + buf_size
 };
 extern "C" ABG_API input_t* pattern_input_new(void);
 

@@ -453,6 +453,7 @@ ABG_API long abh_pattern_selftest(int sfmt, int sample_rate, size_t fft_size, co
     size_t pos = 0;
     const size_t total = block_len * (size_t)repeat;
     int idle_ms = 0;
+    bool lapped = false;  // the source has overwritten bytes not yet read: from then on the byte positions no longer line up
     while (idle_ms < 2000) {
         size_t available;
         pthread_mutex_lock(&in->buffer_lock);
@@ -465,11 +466,18 @@ ABG_API long abh_pattern_selftest(int sfmt, int sample_rate, size_t fft_size, co
             continue;
         }
         idle_ms = 0;
-        if (in->overflow_count == 0) {  // after an overflow the byte positions no longer line up: only count from then on
+        if (!lapped) {
+            long miss = 0;
             for (size_t k = 0; k < available; k++) {
                 const unsigned char got = in->buffer[(in->bufs + k) % in->buf_size];
-                if (got != block[(pos + k) % block_len]) bad++;
+                if (got != block[(pos + k) % block_len]) miss++;
             }
+            // A paced source may lap the ring while the bytes are compared, and overflow_count misses a lap past slot 0.
+            // An append that overwrote any of them stored `written` before it took the ring lock, so it is seen under that lock.
+            pthread_mutex_lock(&in->buffer_lock);
+            lapped = in->overflow_count > 0 || __atomic_load_n(&dd->written, __ATOMIC_ACQUIRE) > pos + in->buf_size;
+            pthread_mutex_unlock(&in->buffer_lock);
+            if (!lapped) bad += miss;
         }
         pos += available;
         in->bufs = (in->bufs + available) % in->buf_size;  // not under the lock, like rtl_airband.cpp:669

@@ -65,6 +65,7 @@ void* pattern_rx_thread(void* ctx) {
         }
         const size_t off = sent % dd->block_len;
         n = std::min(n, dd->block_len - off);  // one append never straddles the block end
+        __atomic_store_n(&dd->written, sent + n, __ATOMIC_RELEASE);
         circbuffer_append(input, const_cast<unsigned char*>(dd->block + off), n);
         sent += n;
     }

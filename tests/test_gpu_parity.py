@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 import oracle_py as op
+import reference_outputs as ro
 from airband_b200 import config as cm
 from airband_b200 import lib
 from airband_b200 import workloads as wl
@@ -52,8 +53,9 @@ def test_case_matches_oracle(name, fft_mode):
 @pytest.mark.parametrize("name", ["am_u8", "nfm_s16", "am_bw_f32", "s8_two_devices"])
 def test_case_matches_golden_fixture(name):
     g = np.load(os.path.join(os.path.dirname(__file__), "golden", name + ".npz"))
-    cfg, _ = CASES[name]()
-    raws = [g[f"raw{d}"] for d in range(len(cfg.devices))]
+    cfg, raws = CASES[name]()
+    for d, r in enumerate(raws):
+        assert ro.digest(r) == str(g[f"raw{d}_sha256"]), "seeded generator no longer reproduces the stored input"
     gres, geng = lib.demodulate_all(cfg, raws)
     for d, (gw, gi, ga) in enumerate(gres):
         assert np.array_equal(ga, g[f"axc{d}"])

@@ -1,10 +1,12 @@
-"""Whole-path checks of the oracle itself: restated leaf classes vs the reference's own (bit-identical audio),
-strict vs the reference's -ffast-math flags (spread must sit far inside the 1e-4 parity gate, SURVEY.md §7.5),
-threaded == single-threaded, streaming pushes == one push, and basic signal sanity (the 1 kHz AM tone comes out)."""
+"""Whole-path checks of the oracle itself: restated leaf classes vs the reference's own (bit-identical audio, against
+their stored outputs: tests/reference_outputs.py), strict vs the reference's -ffast-math flags (spread must sit far inside
+the 1e-4 parity gate, SURVEY.md §7.5), threaded == single-threaded, streaming pushes == one push, and basic signal sanity
+(the 1 kHz AM tone comes out)."""
 import numpy as np
 import pytest
 
 import oracle_py as op
+import reference_outputs as ro
 from airband_b200 import workloads as wl
 from cases import CASES
 
@@ -26,20 +28,26 @@ def test_signal_exercises_the_path(name):
     assert opened >= 1, "squelch never opened: case does not exercise demodulation"
 
 
-@pytest.mark.skipif(not op.available("ref"), reason="oracle/_ref not built")
+def pipeline_outputs(name, variant):
+    """Per device: waveout, iq_out, axcindicate and every squelch statistic of every channel (as float64, exact)."""
+    cfg, raws = CASES[name]()
+    res, o = op.run_oracle(cfg, raws, variant)
+    out = {}
+    for d, (wo, iq, ax) in enumerate(res):
+        out.update({f"waveout{d}": wo, f"iq_out{d}": iq, f"axc{d}": ax})
+        out[f"stats{d}"] = np.array([[float(getattr(o.stats(d, c), f)) for f, _ in o.stats(d, c)._fields_] for c in range(wo.shape[0])])
+    return out
+
+
+def record_reference(out: dict) -> None:
+    """What the original leaf classes compute for every case (tests/golden/make_golden.py)."""
+    for name in CASES:
+        ro.record(out, f"pipeline/{name}", pipeline_outputs(name, "ref"))
+
+
 @pytest.mark.parametrize("name", list(CASES))
 def test_restated_equals_reference_leaf(name):
-    cfg, raws = CASES[name]()
-    ra, oa = op.run_oracle(cfg, raws, "restated")
-    rb, ob = op.run_oracle(cfg, raws, "ref")
-    for d, ((wa, ia, xa), (wb, ib, xb)) in enumerate(zip(ra, rb)):
-        assert np.array_equal(wa.view(np.uint32), wb.view(np.uint32))
-        assert np.array_equal(ia.view(np.uint64), ib.view(np.uint64))
-        assert np.array_equal(xa, xb)
-        for c in range(wa.shape[0]):
-            sa, sb = oa.stats(d, c), ob.stats(d, c)
-            for f, _ in sa._fields_:
-                assert getattr(sa, f) == getattr(sb, f), (d, c, f)
+    ro.check(f"pipeline/{name}", pipeline_outputs(name, "restated"))
 
 
 @pytest.mark.parametrize("name", ["am_u8", "nfm_s16", "am_bw_f32"])

@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 
 import oracle_py as op
+import reference_outputs as ro
 from airband_b200 import config as cm
 from airband_b200 import workloads as wl
 
@@ -43,10 +44,7 @@ def _run(cfg, freqs, visits, raw, variant, nb=4, configure=True):
     return np.concatenate(out, 1), np.concatenate(ax, 0), stats
 
 
-@pytest.mark.parametrize("variant", ["restated", "ref"])
-def test_single_entry_list_is_the_plain_channel(variant):
-    if not op.available(variant):
-        pytest.skip("oracle variant not built")
+def single_entry_outputs(variant):
     cfg, freqs = _setup()
     raw = wl.synth_iq(cfg, 0, wl.samples_for_batches(cfg, 0, 12), key_on_s=1.2, key_off_s=0.2, amplitude=0.2)
     plain_cfg = cm.Config(fft_size=cfg.fft_size, wave_rate=cfg.wave_rate,
@@ -54,6 +52,16 @@ def test_single_entry_list_is_the_plain_channel(variant):
     a, xa, _ = _run(plain_cfg, freqs, [0, 0, 0], raw, variant, configure=False)
     b, xb, _ = _run(cfg, [freqs[0]], [0, 0, 0], raw, variant)
     c, xc, _ = _run(cfg, freqs, [0, 0, 0], raw, variant)        # other entries exist but are never selected
+    return {"plain": a, "plain_axc": xa, "single": b, "single_axc": xb, "unselected": c, "unselected_axc": xc}
+
+
+@pytest.mark.parametrize("variant", ["restated", "ref"])
+def test_single_entry_list_is_the_plain_channel(variant):
+    # "ref": the restated runs must also equal, bit for bit, what the original leaf classes computed in them (stored)
+    out = single_entry_outputs("restated")
+    if variant == "ref":
+        ro.check("scan_single_entry", out)
+    a, xa, b, xb, c, xc = (out[k] for k in ("plain", "plain_axc", "single", "single_axc", "unselected", "unselected_axc"))
     assert np.array_equal(a.view(np.uint32), b.view(np.uint32)) and np.array_equal(xa, xb)
     assert np.array_equal(a.view(np.uint32), c.view(np.uint32)) and np.array_equal(xa, xc)
 
@@ -77,11 +85,19 @@ def test_entries_keep_their_own_state():
     assert not np.array_equal(w_, w2)
 
 
-@pytest.mark.skipif(not op.available("ref"), reason="oracle/_ref not built")
-def test_scan_restated_equals_reference_leaf():
+def scan_outputs(variant):
     cfg, freqs = _setup()
     visits = [0, 1, 2, 1, 0, 2, 2, 0]
     raw = wl.synth_iq(cfg, 0, wl.samples_for_batches(cfg, 0, 4 * len(visits)), key_on_s=1.2, key_off_s=0.2, amplitude=0.2)
-    a, xa, sa = _run(cfg, freqs, visits, raw, "restated")
-    b, xb, sb = _run(cfg, freqs, visits, raw, "ref")
-    assert np.array_equal(a.view(np.uint32), b.view(np.uint32)) and np.array_equal(xa, xb) and sa == sb
+    w_, ax, stats = _run(cfg, freqs, visits, raw, variant)
+    return {"waveout": w_, "axc": ax, "stats": np.array(stats, np.int64)}
+
+
+def record_reference(out: dict) -> None:
+    """What the original leaf classes compute in scan mode (tests/golden/make_golden.py)."""
+    ro.record(out, "scan", scan_outputs("ref"))
+    ro.record(out, "scan_single_entry", single_entry_outputs("ref"))
+
+
+def test_scan_restated_equals_reference_leaf():
+    ro.check("scan", scan_outputs("restated"))

@@ -12,7 +12,7 @@
  *
  * Conventions: every function returns 0 on success and a negative ABG_E* code on failure (the VideoCore engine
  * uses -1/-2/-3 the same way, reference src/rtl_airband.cpp:296-310); abg_last_error() gives the text the caller
- * passes to log(LOG_CRIT, ...) before error().  All buffers are caller-owned host memory unless named dev_*.
+ * passes to log(LOG_CRIT, ...) before error().  All buffers are caller-owned host memory unless named dev_* or d_*.
  * No CPU fallback exists: without a CUDA device abg_create() fails with ABG_ENODEV.
  */
 #ifndef AIRBAND_B200_H
@@ -220,6 +220,38 @@ ABG_API int abg_fetch_mixer_batch(abg_engine* e, int mixer, float* left, float* 
 /* Device pointers to the partial sums of the LATEST run, for a cross-GPU reduction when a mixer's inputs are sharded
  * over several engines: sums float[max_batches_per_run][n_mixers][2][WAVE_BATCH], flags int32[max_batches_per_run][n_mixers]. */
 ABG_API int abg_mixer_device_buffers(abg_engine* e, float** dev_sums, int32_t** dev_flags);
+
+/* ---- GPU-resident I/O (not part of the reference surface) ---------------------------------------------------------
+ * For callers whose IQ is already in GPU memory (GPUDirect capture, a GPU-side DDC) and whose consumers run on the GPU.
+ * Every call here is ordered on the caller's CUDA stream (cudaStream_t passed as void*, NULL = the legacy default
+ * stream) and none of them blocks the host.  All d_* pointers are device memory on the engine's GPU. */
+enum { ABG_RESULTS_HOST = 0, ABG_RESULTS_DEVICE = 1 };
+/* abg_push with a device-memory source: same ring-format bytes, whole complex samples, ABG_EOVERFLOW rule and buffer
+ * compaction.  The engine's ingest stream first waits for the work enqueued so far on cuda_stream, then copies device to
+ * device.  Host pointers and memory on another GPU are rejected with ABG_EINVAL.  abg_push and abg_push_device may be
+ * mixed on one device; the bytes follow each other in call order.  The source must stay unmodified until
+ * abg_ingest_join (or abg_ingest_sync) has covered the push. */
+ABG_API int abg_push_device(abg_engine* e, int dev, const void* d_iq, size_t nbytes, void* cuda_stream);
+/* Make cuda_stream wait until every push so far has been read out of the caller's memory: the non-blocking
+ * counterpart of abg_ingest_sync.  Work the caller enqueues on cuda_stream afterwards may overwrite pushed sources. */
+ABG_API int abg_ingest_join(abg_engine* e, void* cuda_stream);
+/* Where the result slots live: ABG_RESULTS_HOST (default, page-locked host memory) or ABG_RESULTS_DEVICE (HBM).  Only
+ * before the first run (ABG_EINVAL afterwards).  abg_fetch_batch(es) and abg_fetch_mixer_batch keep working in device
+ * mode (they copy out of the device slot); the *_device fetches below need it. */
+ABG_API int abg_set_result_location(abg_engine* e, int where);
+/* Pop up to max_batches finished batches of one device (count taken from the engine's bookkeeping, no wait for the GPU)
+ * and write them on cuda_stream in abg_fetch_batches' layouts: d_waveout[n][C][WAVE_BATCH], d_iq_out[n][C][2*WAVE_BATCH]
+ * (may be NULL; zero-filled when no channel has I/Q outputs), d_axcindicate[n][C] (may be NULL).  Returns n. */
+ABG_API int abg_fetch_batches_device(abg_engine* e, int dev, int max_batches, float* d_waveout, float* d_iq_out, char* d_axcindicate,
+                                     void* cuda_stream);
+/* Pop n_batches batches of EVERY device in one launch, in engine-global channel order: d_waveout[n][G][WAVE_BATCH],
+ * d_iq_out[n][G][2*WAVE_BATCH], d_axcindicate[n][G] (G = all channels of the engine).  ABG_EINVAL, popping nothing, if
+ * some device has fewer than n_batches finished batches. */
+ABG_API int abg_fetch_all_device(abg_engine* e, int n_batches, float* d_waveout, float* d_iq_out, char* d_axcindicate, void* cuda_stream);
+/* Pop up to max_batches finished batches of ALL mixers at once: d_left_right[n][n_mixers][2][WAVE_BATCH],
+ * d_has_signal[n][n_mixers] (may be NULL).  ABG_EINVAL if a mixer was popped on its own (abg_fetch_mixer_batch) and the
+ * mixers are not at the same batch.  Returns n. */
+ABG_API int abg_fetch_mixer_batches_device(abg_engine* e, int max_batches, float* d_left_right, int32_t* d_has_signal, void* cuda_stream);
 
 /* ---- stage taps for tests ---------------------------------------------------------------------------------- */
 /* Run conversion + window + FFT on one frame of `dev`'s format and return the full spectrum in natural bin order

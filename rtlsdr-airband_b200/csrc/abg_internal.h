@@ -212,3 +212,19 @@ struct K2Export {
     size_t stride;             // nbmax * WAVE_BATCH
 };
 cudaError_t abg_launch_k2_tail(const K2Launch& L, const K2Export& X, cudaStream_t s);
+
+// device-resident result fetches (export_device.cu): one launch copies a list of rectangular blocks out of the
+// channel-major result slots in HBM into the caller's batch-major buffers.  Block k copies rows x row_bytes from
+// src (row pitch src_pitch) to dst (row pitch dst_pitch); src == null writes zeros.
+struct GatherCopy {
+    const unsigned char* src;
+    unsigned char* dst;
+    long long src_pitch, dst_pitch;
+    int32_t rows, row_bytes;
+};
+#define ABG_GATHER_MAX 96  // blocks per launch: the list is passed by value and stays below the 4 KB parameter limit
+struct GatherList {
+    int32_t n, max_rows;
+    GatherCopy c[ABG_GATHER_MAX];
+};
+cudaError_t abg_launch_gather(const GatherList& L, cudaStream_t s);

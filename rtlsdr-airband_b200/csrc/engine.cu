@@ -262,15 +262,20 @@ struct Group {
     int tc_tables = 0;
 };
 
+// One run's results.  Page-locked host memory by default; HBM after abg_set_result_location(ABG_RESULTS_DEVICE).
 struct Slot {
-    float* wout = nullptr;    // pinned [G][nbmax*B]
-    float* iqout = nullptr;   // pinned [G][nbmax*B][2] or null
-    unsigned char* axc = nullptr;  // pinned [nbmax][Gp]
-    float* mix = nullptr;     // pinned [nbmax][n_mixers][2][B]
-    int32_t* mixflag = nullptr;  // pinned [nbmax][n_mixers]
+    float* wout = nullptr;    // [G][nbmax*B]
+    float* iqout = nullptr;   // [G][nbmax*B][2] or null
+    unsigned char* axc = nullptr;  // [nbmax][Gp]
+    float* mix = nullptr;     // [nbmax][n_mixers][2][B]
+    int32_t* mixflag = nullptr;  // [nbmax][n_mixers]
     int mix_pending = 0;
     cudaEvent_t done = nullptr;
     int pending = 0;          // unfetched device-batches referencing this slot
+    // device mode: recorded on the caller's stream after the gather of a device fetch that read this slot; a later
+    // run's mixer and export kernels wait for it before they overwrite the slot
+    cudaEvent_t released = nullptr;
+    bool release_pending = false;
 };
 
 }  // namespace
@@ -307,6 +312,8 @@ struct abg_engine {
     cudaStream_t stream_b = nullptr; // stream B: K2, mixers, result copies, tail copy
     cudaStream_t stream_c = nullptr; // stream C: ingest (abg_push host->device copies, buffer compaction)
     cudaEvent_t ev_ingest = nullptr; // last ingest operation
+    cudaEvent_t ev_caller = nullptr; // abg_push_device: the caller's stream up to the push
+    int results_where = ABG_RESULTS_HOST;
     bool ingest_dirty = false;
     cudaEvent_t ev_k1[2] = {nullptr, nullptr}, ev_k2[2] = {nullptr, nullptr};
     uint64_t run_index = 0;
@@ -342,11 +349,48 @@ struct abg_engine {
 
 namespace {
 
+// result slot memory: page-locked host memory, or HBM in device mode
+cudaError_t result_alloc(const abg_engine* e, void** p, size_t bytes) {
+    return e->results_where == ABG_RESULTS_DEVICE ? cudaMalloc(p, bytes) : cudaMallocHost(p, bytes);
+}
+template <typename T>
+void result_free(const abg_engine* e, T*& p) {
+    if (p) {
+        if (e->results_where == ABG_RESULTS_DEVICE) cudaFree(p);
+        else cudaFreeHost(p);
+    }
+    p = nullptr;
+}
+int alloc_slot_results(abg_engine* e) {
+    const size_t GB = (size_t)std::max(e->G, 1) * e->nbmax * e->B;
+    for (auto& s : e->slots) {
+        CU(result_alloc(e, (void**)&s.wout, sizeof(float) * GB));
+        if (e->any_iq_out) CU(result_alloc(e, (void**)&s.iqout, sizeof(float2) * GB));
+        CU(result_alloc(e, (void**)&s.axc, (size_t)e->nbmax * e->Gp));
+    }
+    return ABG_OK;
+}
+int alloc_slot_mixers(abg_engine* e) {
+    const size_t nsum = (size_t)e->nbmax * e->n_mixers * 2 * e->B;
+    for (auto& s : e->slots) {
+        CU(result_alloc(e, (void**)&s.mix, sizeof(float) * nsum));
+        CU(result_alloc(e, (void**)&s.mixflag, sizeof(int32_t) * (size_t)e->nbmax * e->n_mixers));
+    }
+    return ABG_OK;
+}
+void free_slot_results(abg_engine* e) {
+    for (auto& s : e->slots) {
+        result_free(e, s.wout); result_free(e, s.iqout); result_free(e, s.axc); result_free(e, s.mix); result_free(e, s.mixflag);
+    }
+}
+
 void engine_free(abg_engine* e) {
     if (!e) return;
     cudaSetDevice(e->cuda_dev);
     if (e->stream) cudaStreamSynchronize(e->stream);
     if (e->stream_b) cudaStreamSynchronize(e->stream_b);
+    for (auto& s : e->slots)  // device fetches still reading a slot on a caller's stream
+        if (s.release_pending) cudaEventSynchronize(s.released);
     for (auto& d : e->dev) {
         for (int i = 0; i < 2; i++)
             if (d.raw[i]) cudaFree(d.raw[i]);
@@ -365,13 +409,10 @@ void engine_free(abg_engine* e) {
     if (e->d_k2) cudaFree(e->d_k2);
     for (auto& sc : e->scan)
         if (sc.stash) cudaFree(sc.stash);
+    free_slot_results(e);
     for (auto& s : e->slots) {
-        if (s.wout) cudaFreeHost(s.wout);
-        if (s.iqout) cudaFreeHost(s.iqout);
-        if (s.axc) cudaFreeHost(s.axc);
-        if (s.mix) cudaFreeHost(s.mix);
-        if (s.mixflag) cudaFreeHost(s.mixflag);
         if (s.done) cudaEventDestroy(s.done);
+        if (s.released) cudaEventDestroy(s.released);
     }
     for (auto& row : e->tl)
         for (auto& ev : row)
@@ -386,6 +427,7 @@ void engine_free(abg_engine* e) {
         cudaStreamDestroy(e->stream_c);
     }
     if (e->ev_ingest) cudaEventDestroy(e->ev_ingest);
+    if (e->ev_caller) cudaEventDestroy(e->ev_caller);
     if (e->own_stream && e->stream) cudaStreamDestroy(e->stream);
     delete e;
 }
@@ -686,6 +728,7 @@ int build(abg_engine* e, const abg_config* cfg, const abg_options* opt) {
         for (auto& ev : row) CU(cudaEventCreate(&ev));
     CU(cudaStreamCreateWithFlags(&e->stream_c, cudaStreamNonBlocking));
     CU(cudaEventCreateWithFlags(&e->ev_ingest, cudaEventDisableTiming));
+    CU(cudaEventCreateWithFlags(&e->ev_caller, cudaEventDisableTiming));
     for (auto& d : e->dev)
         if (d.has_afc) e->any_afc = true;
     {
@@ -779,10 +822,12 @@ int build(abg_engine* e, const abg_config* cfg, const abg_options* opt) {
     e->h_k2.assign(e->dev.size(), K2Dev{});
     e->slots.resize(3);
     for (auto& s : e->slots) {
-        CU(cudaMallocHost((void**)&s.wout, sizeof(float) * (size_t)std::max(G, 1) * e->nbmax * B));
-        if (e->any_iq_out) CU(cudaMallocHost((void**)&s.iqout, sizeof(float2) * (size_t)std::max(G, 1) * e->nbmax * B));
-        CU(cudaMallocHost((void**)&s.axc, (size_t)e->nbmax * Gp));
         CU(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&s.released, cudaEventDisableTiming));
+    }
+    {
+        const int rc = alloc_slot_results(e);
+        if (rc != ABG_OK) return rc;
     }
     CU(cudaStreamSynchronize(e->stream));
     return ABG_OK;
@@ -888,6 +933,8 @@ int enqueue_run(abg_engine* e, const std::vector<int>& nb, bool resident, bool q
     if (er != cudaSuccess) return fail(ABG_ECUDA, "K2 launch failed: %s", cudaGetErrorString(er));
     e->launches++;
     CU(cudaEventRecord(tl[3], sb));
+    // device mode: a device fetch may still be copying this slot's previous contents on the caller's stream
+    if (queue_outputs && e->slots[slot].release_pending) CU(cudaStreamWaitEvent(sb, e->slots[slot].released, 0));
     // ---- mixers: sums over the just-finished batches, before the tail copy (output.cpp:533-535 -> mixer.cpp) ----
     if (e->n_mixers > 0) {
         MixLaunch M{};
@@ -949,6 +996,92 @@ int enqueue_run(abg_engine* e, const std::vector<int>& nb, bool resident, bool q
     return ABG_OK;
 }
 
+// Append nbytes at the end of a device's raw stream on the ingest stream (stream C), compacting first when they do
+// not fit behind the buffered bytes.  abg_push (host source) and abg_push_device (device source) differ only in `kind`.
+int push_bytes(abg_engine* e, int dev, const void* iq, size_t nbytes, cudaMemcpyKind kind, const char* who) {
+    Device& d = e->dev[dev];
+    if (d.fill + nbytes > d.cap) {
+        // compact: move the unconsumed tail to the front of the other buffer.  Ingest runs on its own stream so that
+        // host->device copies overlap K1; the other buffer may still be read by the most recent K1, so wait for it.
+        const size_t keep_from = d.consumed & ~(size_t)15;  // keep the copy 16-byte aligned on both sides
+        const size_t rem = d.fill - keep_from;
+        if (rem + nbytes > d.cap) {
+            return fail(ABG_EOVERFLOW, "%s: device %d input buffer overflow (%zu buffered + %zu new > %zu)", who, dev, d.fill - d.consumed, nbytes, d.cap);
+        }
+        // the destination buffer was last read by a K1 launched before the previous compaction: with at least one run since
+        // then that is run_index-2 or older, so the copy overlaps the K1 that is reading the current buffer right now
+        if (d.runs_since_compaction >= 1) {
+            if (e->run_index >= 2) CU(cudaStreamWaitEvent(e->stream_c, e->ev_k1[(e->run_index - 2) & 1], 0));
+        } else if (e->run_index >= 1) {
+            CU(cudaStreamWaitEvent(e->stream_c, e->ev_k1[(e->run_index - 1) & 1], 0));
+        }
+        d.runs_since_compaction = 0;
+        CU(cudaMemcpyAsync(d.raw[d.cur ^ 1], d.raw[d.cur] + keep_from, rem, cudaMemcpyDeviceToDevice, e->stream_c));
+        d.cur ^= 1;
+        d.fill = rem;
+        d.consumed -= keep_from;
+    }
+    CU(cudaMemcpyAsync(d.raw[d.cur] + d.fill, iq, nbytes, kind, e->stream_c));
+    e->ingest_dirty = true;
+    d.fill += nbytes;
+    return ABG_OK;
+}
+
+// ---- device-resident result fetches -------------------------------------------------------------------------------
+// The blocks of one batch: channels [g_begin, g_begin + nch) of batch b (of its run) in slot s go to channel offset dst_ch
+// of the caller's batch-major buffers (audio and I/Q rows of WAVE_BATCH samples, one flag byte per channel).
+void gather_batch(const abg_engine* e, std::vector<GatherCopy>& cps, const Slot& s, int b, int g_begin, int nch, size_t dst_ch, float* d_wo,
+                  float* d_iq, char* d_axc) {
+    const size_t B = (size_t)e->B, stride = (size_t)e->nbmax * e->B;
+    const size_t src0 = (size_t)g_begin * stride + (size_t)b * B;
+    if (d_wo)
+        cps.push_back({reinterpret_cast<const unsigned char*>(s.wout + src0), reinterpret_cast<unsigned char*>(d_wo + dst_ch * B),
+                       (long long)(sizeof(float) * stride), (long long)(sizeof(float) * B), nch, (int32_t)(sizeof(float) * B)});
+    if (d_iq)  // no channel with I/Q outputs: zeros, like the host path
+        cps.push_back({s.iqout ? reinterpret_cast<const unsigned char*>(s.iqout + 2 * src0) : nullptr, reinterpret_cast<unsigned char*>(d_iq + dst_ch * 2 * B),
+                       (long long)(sizeof(float2) * stride), (long long)(sizeof(float2) * B), nch, (int32_t)(sizeof(float2) * B)});
+    if (d_axc)
+        cps.push_back({s.axc + (size_t)b * e->Gp + g_begin, reinterpret_cast<unsigned char*>(d_axc + dst_ch), nch, nch, 1, nch});
+}
+
+// Enqueue the gather on the caller's stream.  It first waits for the runs that filled the slots, and for earlier device
+// fetches from them (so that the release event recorded afterwards covers every reader of the slot, whatever stream it
+// used); enqueue_run makes the export of a later run into one of these slots wait for that release event.
+int gather_launch(abg_engine* e, const std::vector<GatherCopy>& cps, const std::vector<int>& slots, cudaStream_t cs) {
+    for (int k : slots) {
+        const Slot& s = e->slots[k];
+        CU(cudaStreamWaitEvent(cs, s.done, 0));
+        if (s.release_pending) CU(cudaStreamWaitEvent(cs, s.released, 0));
+    }
+    for (size_t i0 = 0; i0 < cps.size(); i0 += ABG_GATHER_MAX) {
+        GatherList L;
+        L.n = (int32_t)std::min<size_t>(ABG_GATHER_MAX, cps.size() - i0);
+        L.max_rows = 0;
+        for (int i = 0; i < L.n; i++) {
+            L.c[i] = cps[i0 + i];
+            L.max_rows = std::max(L.max_rows, L.c[i].rows);
+        }
+        const cudaError_t er = abg_launch_gather(L, cs);
+        if (er != cudaSuccess) return fail(ABG_ECUDA, "result gather launch failed: %s", cudaGetErrorString(er));
+        e->launches++;
+    }
+    for (int k : slots) {
+        Slot& s = e->slots[k];
+        CU(cudaEventRecord(s.released, cs));
+        s.release_pending = true;
+    }
+    return ABG_OK;
+}
+
+void note_slot(std::vector<int>& used, int slot) {
+    if (std::find(used.begin(), used.end(), slot) == used.end()) used.push_back(slot);
+}
+
+int need_device_results(const abg_engine* e, const char* who) {
+    if (e->results_where == ABG_RESULTS_DEVICE) return ABG_OK;
+    return fail(ABG_EINVAL, "%s: results are in host memory; call abg_set_result_location(ABG_RESULTS_DEVICE) before the first run", who);
+}
+
 }  // namespace
 
 // =========================================================================================================================
@@ -1004,30 +1137,33 @@ int abg_push(abg_engine* e, int dev, const void* iq, size_t nbytes) {
     if (nbytes == 0) return ABG_OK;
     if (nbytes % d.bpc) return fail(ABG_EINVAL, "abg_push: %zu bytes is not a whole number of complex samples", nbytes);
     cudaSetDevice(e->cuda_dev);
-    if (d.fill + nbytes > d.cap) {
-        // compact: move the unconsumed tail to the front of the other buffer.  Ingest runs on its own stream so that
-        // host->device copies overlap K1; the other buffer may still be read by the most recent K1, so wait for it.
-        const size_t keep_from = d.consumed & ~(size_t)15;  // keep the copy 16-byte aligned on both sides
-        const size_t rem = d.fill - keep_from;
-        if (rem + nbytes > d.cap) {
-            return fail(ABG_EOVERFLOW, "abg_push: device %d input buffer overflow (%zu buffered + %zu new > %zu)", dev, d.fill - d.consumed, nbytes, d.cap);
-        }
-        // the destination buffer was last read by a K1 launched before the previous compaction: with at least one run since
-        // then that is run_index-2 or older, so the copy overlaps the K1 that is reading the current buffer right now
-        if (d.runs_since_compaction >= 1) {
-            if (e->run_index >= 2) CU(cudaStreamWaitEvent(e->stream_c, e->ev_k1[(e->run_index - 2) & 1], 0));
-        } else if (e->run_index >= 1) {
-            CU(cudaStreamWaitEvent(e->stream_c, e->ev_k1[(e->run_index - 1) & 1], 0));
-        }
-        d.runs_since_compaction = 0;
-        CU(cudaMemcpyAsync(d.raw[d.cur ^ 1], d.raw[d.cur] + keep_from, rem, cudaMemcpyDeviceToDevice, e->stream_c));
-        d.cur ^= 1;
-        d.fill = rem;
-        d.consumed -= keep_from;
+    return push_bytes(e, dev, iq, nbytes, cudaMemcpyHostToDevice, "abg_push");
+}
+
+int abg_push_device(abg_engine* e, int dev, const void* d_iq, size_t nbytes, void* cuda_stream) {
+    if (dev < 0 || dev >= (int)e->dev.size()) return fail(ABG_ERANGE, "abg_push_device: device %d out of range", dev);
+    Device& d = e->dev[dev];
+    if (nbytes == 0) return ABG_OK;
+    if (nbytes % d.bpc) return fail(ABG_EINVAL, "abg_push_device: %zu bytes is not a whole number of complex samples", nbytes);
+    if (!d_iq) return fail(ABG_EINVAL, "abg_push_device: null source");
+    cudaSetDevice(e->cuda_dev);
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, d_iq) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(ABG_EINVAL, "abg_push_device: %p is not a CUDA allocation", d_iq);
     }
-    CU(cudaMemcpyAsync(d.raw[d.cur] + d.fill, iq, nbytes, cudaMemcpyHostToDevice, e->stream_c));
-    e->ingest_dirty = true;
-    d.fill += nbytes;
+    if (a.type != cudaMemoryTypeDevice || a.device != e->cuda_dev)
+        return fail(ABG_EINVAL, "abg_push_device: source must be device memory on GPU %d (memory type %d on device %d)", e->cuda_dev, (int)a.type, a.device);
+    // what the caller enqueued on its stream so far (e.g. the kernel that produced the samples) comes first
+    CU(cudaEventRecord(e->ev_caller, (cudaStream_t)cuda_stream));
+    CU(cudaStreamWaitEvent(e->stream_c, e->ev_caller, 0));
+    return push_bytes(e, dev, d_iq, nbytes, cudaMemcpyDeviceToDevice, "abg_push_device");
+}
+
+int abg_ingest_join(abg_engine* e, void* cuda_stream) {
+    cudaSetDevice(e->cuda_dev);
+    CU(cudaEventRecord(e->ev_ingest, e->stream_c));
+    CU(cudaStreamWaitEvent((cudaStream_t)cuda_stream, e->ev_ingest, 0));
     return ABG_OK;
 }
 
@@ -1082,6 +1218,20 @@ int abg_fetch_batch(abg_engine* e, int dev, float* waveout, float* iq_out, char*
     if (e->tc_status && e->tc_status[0]) return fail(ABG_ECUDA, "tensor-core K1 pipeline stalled (wait code %d); results of that run are invalid", e->tc_status[0]);
     const int B = e->B;
     const size_t stride = (size_t)e->nbmax * B;
+    if (e->results_where == ABG_RESULTS_DEVICE) {  // the same bytes, copied out of the slot in HBM
+        const size_t g0 = (size_t)d.g0, off = (size_t)r.second * B;
+        if (waveout) CU(cudaMemcpy2D(waveout, sizeof(float) * B, s.wout + g0 * stride + off, sizeof(float) * stride, sizeof(float) * B, d.C, cudaMemcpyDeviceToHost));
+        if (iq_out) {
+            if (s.iqout)
+                CU(cudaMemcpy2D(iq_out, sizeof(float2) * B, s.iqout + 2 * (g0 * stride + off), sizeof(float2) * stride, sizeof(float2) * B, d.C, cudaMemcpyDeviceToHost));
+            else
+                memset(iq_out, 0, sizeof(float) * 2 * B * d.C);
+        }
+        if (axcindicate) CU(cudaMemcpy(axcindicate, s.axc + (size_t)r.second * e->Gp + g0, d.C, cudaMemcpyDeviceToHost));
+        d.ready.pop_front();
+        s.pending--;
+        return 1;
+    }
     for (int c = 0; c < d.C; c++) {
         const size_t g = (size_t)d.g0 + c;
         if (waveout) memcpy(waveout + (size_t)c * B, s.wout + g * stride + (size_t)r.second * B, sizeof(float) * B);
@@ -1367,9 +1517,9 @@ int abg_mixers_configure(abg_engine* e, int n_mixers, const int32_t* input_offse
     }
     e->mix_offsets.free(); e->mix_inputs.free(); e->mix_sums.free(); e->mix_flags.free();
     for (auto& s : e->slots) {
-        if (s.mix) cudaFreeHost(s.mix);
-        if (s.mixflag) cudaFreeHost(s.mixflag);
-        s.mix = nullptr; s.mixflag = nullptr;
+        if (s.release_pending) CU(cudaEventSynchronize(s.released));
+        result_free(e, s.mix);
+        result_free(e, s.mixflag);
     }
     e->n_mixers = n_mixers;
     e->mix_fetched.assign(n_mixers, 0);
@@ -1381,11 +1531,7 @@ int abg_mixers_configure(abg_engine* e, int n_mixers, const int32_t* input_offse
     if (total) CU(cudaMemcpy(e->mix_inputs.p, mi.data(), sizeof(MixInput) * total, cudaMemcpyHostToDevice));
     CU(cudaMemset(e->mix_sums.p, 0, sizeof(float) * nsum));
     CU(cudaMemset(e->mix_flags.p, 0, sizeof(int32_t) * (size_t)e->nbmax * n_mixers));
-    for (auto& s : e->slots) {
-        CU(cudaMallocHost((void**)&s.mix, sizeof(float) * nsum));
-        CU(cudaMallocHost((void**)&s.mixflag, sizeof(int32_t) * (size_t)e->nbmax * n_mixers));
-    }
-    return ABG_OK;
+    return alloc_slot_mixers(e);
 }
 
 int abg_fetch_mixer_batch(abg_engine* e, int mixer, float* left, float* right, int* has_signal) {
@@ -1398,9 +1544,16 @@ int abg_fetch_mixer_batch(abg_engine* e, int mixer, float* left, float* right, i
     CU(cudaEventSynchronize(s.done));
     const int B = e->B;
     const float* base = s.mix + (((size_t)r.second * e->n_mixers + mixer) * 2) * B;
-    if (left) memcpy(left, base, sizeof(float) * B);
-    if (right) memcpy(right, base + B, sizeof(float) * B);
-    if (has_signal) *has_signal = s.mixflag[(size_t)r.second * e->n_mixers + mixer];
+    const int32_t* flag = s.mixflag + (size_t)r.second * e->n_mixers + mixer;
+    if (e->results_where == ABG_RESULTS_DEVICE) {
+        if (left) CU(cudaMemcpy(left, base, sizeof(float) * B, cudaMemcpyDeviceToHost));
+        if (right) CU(cudaMemcpy(right, base + B, sizeof(float) * B, cudaMemcpyDeviceToHost));
+        if (has_signal) CU(cudaMemcpy(has_signal, flag, sizeof(int32_t), cudaMemcpyDeviceToHost));
+    } else {
+        if (left) memcpy(left, base, sizeof(float) * B);
+        if (right) memcpy(right, base + B, sizeof(float) * B);
+        if (has_signal) *has_signal = *flag;
+    }
     e->mix_fetched[mixer]++;
     s.mix_pending--;
     // drop queue entries every mixer has consumed
@@ -1419,6 +1572,113 @@ int abg_mixer_device_buffers(abg_engine* e, float** dev_sums, int32_t** dev_flag
     if (dev_sums) *dev_sums = e->mix_sums.p;
     if (dev_flags) *dev_flags = e->mix_flags.p;
     return ABG_OK;
+}
+
+// ---- GPU-resident I/O ---------------------------------------------------------------------------------------------------
+int abg_set_result_location(abg_engine* e, int where) {
+    if (where != ABG_RESULTS_HOST && where != ABG_RESULTS_DEVICE) return fail(ABG_EINVAL, "abg_set_result_location: unknown location %d", where);
+    if (e->run_index > 0) return fail(ABG_EINVAL, "abg_set_result_location: only valid before the first run");
+    if (where == e->results_where) return ABG_OK;
+    cudaSetDevice(e->cuda_dev);
+    free_slot_results(e);
+    e->results_where = where;
+    int rc = alloc_slot_results(e);
+    if (rc == ABG_OK && e->n_mixers > 0) rc = alloc_slot_mixers(e);
+    return rc;
+}
+
+int abg_fetch_batches_device(abg_engine* e, int dev, int max_batches, float* d_waveout, float* d_iq_out, char* d_axcindicate, void* cuda_stream) {
+    if (dev < 0 || dev >= (int)e->dev.size()) return fail(ABG_ERANGE, "abg_fetch_batches_device: device %d out of range", dev);
+    const int rc0 = need_device_results(e, "abg_fetch_batches_device");
+    if (rc0 != ABG_OK) return rc0;
+    if (max_batches < 0) return fail(ABG_EINVAL, "abg_fetch_batches_device: max_batches %d < 0", max_batches);
+    Device& d = e->dev[dev];
+    const int n = std::min(max_batches, (int)d.ready.size());
+    if (n == 0) return 0;
+    cudaSetDevice(e->cuda_dev);
+    std::vector<GatherCopy> cps;
+    std::vector<int> used;
+    for (int i = 0; i < n; i++) {
+        const std::pair<int, int> r = d.ready[i];
+        gather_batch(e, cps, e->slots[r.first], r.second, d.g0, d.C, (size_t)i * d.C, d_waveout, d_iq_out, d_axcindicate);
+        note_slot(used, r.first);
+    }
+    const int rc = gather_launch(e, cps, used, (cudaStream_t)cuda_stream);
+    if (rc != ABG_OK) return rc;
+    for (int i = 0; i < n; i++) {
+        e->slots[d.ready.front().first].pending--;
+        d.ready.pop_front();
+    }
+    return n;
+}
+
+int abg_fetch_all_device(abg_engine* e, int n_batches, float* d_waveout, float* d_iq_out, char* d_axcindicate, void* cuda_stream) {
+    const int rc0 = need_device_results(e, "abg_fetch_all_device");
+    if (rc0 != ABG_OK) return rc0;
+    if (n_batches < 0) return fail(ABG_EINVAL, "abg_fetch_all_device: n_batches %d < 0", n_batches);
+    const size_t nd = e->dev.size();
+    for (size_t k = 0; k < nd; k++)
+        if ((int)e->dev[k].ready.size() < n_batches)
+            return fail(ABG_EINVAL, "abg_fetch_all_device: device %zu has %zu finished batches, fewer than %d", k, e->dev[k].ready.size(), n_batches);
+    if (n_batches == 0) return 0;
+    cudaSetDevice(e->cuda_dev);
+    std::vector<GatherCopy> cps;
+    std::vector<int> used;
+    for (int i = 0; i < n_batches; i++) {
+        // consecutive devices whose i-th batch sits at the same place of the same slot are one block: their channels are
+        // adjacent in the slot and in the output (with every device in step, one block per batch and array)
+        for (size_t k = 0; k < nd;) {
+            const std::pair<int, int> r = e->dev[k].ready[i];
+            const int g_begin = e->dev[k].g0;
+            int g_end = g_begin + e->dev[k].C;
+            size_t j = k + 1;
+            while (j < nd && e->dev[j].ready[i] == r) g_end += e->dev[j++].C;
+            gather_batch(e, cps, e->slots[r.first], r.second, g_begin, g_end - g_begin, (size_t)i * e->G + g_begin, d_waveout, d_iq_out, d_axcindicate);
+            note_slot(used, r.first);
+            k = j;
+        }
+    }
+    const int rc = gather_launch(e, cps, used, (cudaStream_t)cuda_stream);
+    if (rc != ABG_OK) return rc;
+    for (auto& d : e->dev)
+        for (int i = 0; i < n_batches; i++) {
+            e->slots[d.ready.front().first].pending--;
+            d.ready.pop_front();
+        }
+    return n_batches;
+}
+
+int abg_fetch_mixer_batches_device(abg_engine* e, int max_batches, float* d_left_right, int32_t* d_has_signal, void* cuda_stream) {
+    const int rc0 = need_device_results(e, "abg_fetch_mixer_batches_device");
+    if (rc0 != ABG_OK) return rc0;
+    if (e->n_mixers <= 0) return fail(ABG_EINVAL, "abg_fetch_mixer_batches_device: no mixers configured");
+    if (max_batches < 0) return fail(ABG_EINVAL, "abg_fetch_mixer_batches_device: max_batches %d < 0", max_batches);
+    for (int v : e->mix_fetched)
+        if (v != 0) return fail(ABG_EINVAL, "abg_fetch_mixer_batches_device: mixers were popped one by one (abg_fetch_mixer_batch) and are not at the same batch");
+    const int M = e->n_mixers, n = std::min(max_batches, (int)e->mix_ready.size());
+    if (n == 0) return 0;
+    cudaSetDevice(e->cuda_dev);
+    const size_t B = (size_t)e->B, row = (size_t)M * 2 * B;
+    std::vector<GatherCopy> cps;
+    std::vector<int> used;
+    for (int i = 0; i < n; i++) {
+        const std::pair<int, int> r = e->mix_ready[i];
+        const Slot& s = e->slots[r.first];
+        if (d_left_right)  // [M][2] rows of WAVE_BATCH floats, contiguous on both sides
+            cps.push_back({reinterpret_cast<const unsigned char*>(s.mix + (size_t)r.second * row), reinterpret_cast<unsigned char*>(d_left_right + (size_t)i * row),
+                           (long long)(sizeof(float) * B), (long long)(sizeof(float) * B), 2 * M, (int32_t)(sizeof(float) * B)});
+        if (d_has_signal)
+            cps.push_back({reinterpret_cast<const unsigned char*>(s.mixflag + (size_t)r.second * M), reinterpret_cast<unsigned char*>(d_has_signal + (size_t)i * M),
+                           (long long)(sizeof(int32_t) * M), (long long)(sizeof(int32_t) * M), 1, (int32_t)(sizeof(int32_t) * M)});
+        note_slot(used, r.first);
+    }
+    const int rc = gather_launch(e, cps, used, (cudaStream_t)cuda_stream);
+    if (rc != ABG_OK) return rc;
+    for (int i = 0; i < n; i++) {
+        e->slots[e->mix_ready.front().first].mix_pending -= M;
+        e->mix_ready.pop_front();
+    }
+    return n;
 }
 
 // Host-only (no device needed): the tensor-core K1's plan and coefficient table for one device, exactly as abg_create

@@ -23,7 +23,11 @@ SYMBOLS = [
     "abg_batches_available", "abg_run", "abg_sync", "abg_join", "abg_batches_ready", "abg_fetch_batch", "abg_fetch_batches", "abg_get_stats", "abg_set_bin",
     "abg_resident_load", "abg_run_resident", "abg_set_stream", "abg_launch_count", "abg_mixers_configure",
     "abg_fetch_mixer_batch", "abg_mixer_device_buffers", "abg_debug_frame", "abg_last_run_times", "abg_debug_timeline", "abg_scan_configure", "abg_scan_select", "abg_host_register", "abg_host_unregister", "abg_ingest_sync", "abg_fft_path", "abg_debug_tc_table", "abg_debug_inject_wavein", "abg_debug_k1tc_trace", "abg_debug_k2_stats",
+    "abg_push_device", "abg_ingest_join", "abg_set_result_location", "abg_fetch_batches_device", "abg_fetch_all_device",
+    "abg_fetch_mixer_batches_device",
 ]
+
+RESULTS_HOST, RESULTS_DEVICE = 0, 1  # abg_set_result_location
 
 
 class COptions(C.Structure):
@@ -94,6 +98,12 @@ def load():
     L.abg_debug_inject_wavein.restype, L.abg_debug_inject_wavein.argtypes = i, [vp, i, i, vp]
     L.abg_debug_k1tc_trace.restype, L.abg_debug_k1tc_trace.argtypes = i, [vp]
     L.abg_debug_k2_stats.restype, L.abg_debug_k2_stats.argtypes = i, [vp]
+    L.abg_push_device.restype, L.abg_push_device.argtypes = i, [vp, i, vp, C.c_size_t, vp]
+    L.abg_ingest_join.restype, L.abg_ingest_join.argtypes = i, [vp, vp]
+    L.abg_set_result_location.restype, L.abg_set_result_location.argtypes = i, [vp, i]
+    L.abg_fetch_batches_device.restype, L.abg_fetch_batches_device.argtypes = i, [vp, i, i, vp, vp, vp, vp]
+    L.abg_fetch_all_device.restype, L.abg_fetch_all_device.argtypes = i, [vp, i, vp, vp, vp, vp]
+    L.abg_fetch_mixer_batches_device.restype, L.abg_fetch_mixer_batches_device.argtypes = i, [vp, i, vp, vp, vp]
     L.abg_debug_tc_table.restype = i
     L.abg_debug_tc_table.argtypes = [i, i, i, f, i, vp, i, vp, vp, C.c_size_t, vp, C.POINTER(C.c_double)]
     _LIB = L
@@ -119,6 +129,9 @@ class Engine:
         self.h = h
         self.B = self.L.abg_wave_batch(self.h)
         self.nbmax = max_batches_per_run
+        self.cuda_device = cuda_device  # -1: the CUDA device that was current at creation
+        self.G = sum(len(d.channels) for d in cfg.devices)
+        self._n_mixers = 0
 
     def _chk(self, rc: int) -> int:
         if rc < 0:
@@ -199,6 +212,91 @@ class Engine:
     def set_bin(self, dev: int, chan: int, bin_: int) -> None:
         self._chk(self.L.abg_set_bin(self.h, dev, chan, bin_))
 
+    # ---- GPU-resident I/O (torch CUDA tensors; torch is imported only here) ------------------------------------------
+    # Every method runs on torch.cuda.current_stream() of the engine's GPU and never waits on the host.
+    def results_on_device(self) -> None:
+        """Keep result slots in HBM (ABG_RESULTS_DEVICE); needed by the fetch_*_tensors methods.  Before the first run."""
+        self._chk(self.L.abg_set_result_location(self.h, RESULTS_DEVICE))
+
+    def _torch_device(self):
+        import torch
+        return torch.device("cuda", self.cuda_device if self.cuda_device >= 0 else torch.cuda.current_device())
+
+    def _stream(self) -> int:
+        import torch
+        return torch.cuda.current_stream(self._torch_device()).cuda_stream
+
+    def push_device_ptr(self, dev: int, ptr: int, nbytes: int, stream: Optional[int] = None) -> None:
+        """abg_push_device on raw device memory, ordered after the work enqueued so far on `stream` (default: current)."""
+        self._chk(self.L.abg_push_device(self.h, dev, C.c_void_p(ptr), nbytes, C.c_void_p(self._stream() if stream is None else stream)))
+
+    def ingest_join(self, stream: Optional[int] = None) -> None:
+        self._chk(self.L.abg_ingest_join(self.h, C.c_void_p(self._stream() if stream is None else stream)))
+
+    def push_tensor(self, dev: int, t) -> None:
+        """Push ring-format samples from a contiguous CUDA tensor on the engine's GPU: uint8 for U8 devices, int8 for S8,
+        int16 for S16, float32 or complex64 for F32.  The current stream then waits until the engine has copied the
+        samples out, so the tensor may be overwritten or freed by work enqueued on that stream afterwards."""
+        import torch
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"push_tensor expects a torch.Tensor, got {type(t).__name__}")
+        if not 0 <= dev < len(self.cfg.devices):
+            raise ValueError(f"device {dev} out of range")
+        from .config import SFMT_U8, SFMT_S8, SFMT_S16, SFMT_F32
+        want = {SFMT_U8: (torch.uint8,), SFMT_S8: (torch.int8,), SFMT_S16: (torch.int16,),
+                SFMT_F32: (torch.float32, torch.complex64)}[self.cfg.devices[dev].sfmt]
+        if t.dtype not in want:
+            raise TypeError(f"device {dev} takes {' or '.join(str(w) for w in want)} samples, got {t.dtype}")
+        if not t.is_cuda:
+            raise ValueError("push_tensor expects a CUDA tensor (use push() for host memory)")
+        if not t.is_contiguous():
+            raise ValueError("push_tensor expects a contiguous tensor")
+        if self.cuda_device >= 0 and t.device.index != self.cuda_device:
+            raise ValueError(f"tensor is on cuda:{t.device.index}, the engine on cuda:{self.cuda_device}")
+        stream = torch.cuda.current_stream(t.device).cuda_stream
+        nbytes = t.numel() * t.element_size()
+        self._chk(self.L.abg_push_device(self.h, dev, C.c_void_p(t.data_ptr()), nbytes, C.c_void_p(stream)))
+        self._chk(self.L.abg_ingest_join(self.h, C.c_void_p(stream)))
+
+    def _result_tensors(self, n: int, rows: int, want_iq: bool):
+        import torch
+        dv = self._torch_device()
+        wo = torch.empty((n, rows, self.B), dtype=torch.float32, device=dv)
+        iq = torch.empty((n, rows, self.B), dtype=torch.complex64, device=dv) if want_iq else None
+        ax = torch.empty((n, rows), dtype=torch.uint8, device=dv)
+        return wo, iq, ax
+
+    @staticmethod
+    def _tptr(t):
+        return None if t is None else C.c_void_p(t.data_ptr())
+
+    def fetch_tensors(self, dev: int, max_batches: int, want_iq: bool = True, out=None):
+        """Pop up to max_batches finished batches of a device into CUDA tensors: (waveout float32[n, C, B],
+        iq_out complex64[n, C, B] or None, axcindicate uint8[n, C]).  `out` = preallocated tensors of at least that size."""
+        n = min(max_batches, self.batches_ready(dev))
+        Cn = len(self.cfg.devices[dev].channels)
+        wo, iq, ax = out if out is not None else self._result_tensors(n, Cn, want_iq)
+        got = self._chk(self.L.abg_fetch_batches_device(self.h, dev, n, self._tptr(wo), self._tptr(iq), self._tptr(ax),
+                                                        C.c_void_p(self._stream())))
+        return wo[:got], (iq[:got] if iq is not None else None), ax[:got]
+
+    def fetch_all_tensors(self, n_batches: int, want_iq: bool = True, out=None):
+        """Pop n_batches batches of every device in one launch: (waveout float32[n, G, B], iq_out complex64[n, G, B] or
+        None, axcindicate uint8[n, G]), G = every channel of the engine in device order."""
+        wo, iq, ax = out if out is not None else self._result_tensors(n_batches, self.G, want_iq)
+        got = self._chk(self.L.abg_fetch_all_device(self.h, n_batches, self._tptr(wo), self._tptr(iq), self._tptr(ax),
+                                                    C.c_void_p(self._stream())))
+        return wo[:got], (iq[:got] if iq is not None else None), ax[:got]
+
+    def fetch_mixer_tensors(self, max_batches: int):
+        """Pop up to max_batches batches of every mixer: (left_right float32[n, n_mixers, 2, B], has_signal int32[n, n_mixers])."""
+        import torch
+        M, dv = self._n_mixers, self._torch_device()
+        lr = torch.empty((max_batches, M, 2, self.B), dtype=torch.float32, device=dv)
+        hs = torch.empty((max_batches, M), dtype=torch.int32, device=dv)
+        got = self._chk(self.L.abg_fetch_mixer_batches_device(self.h, max_batches, self._tptr(lr), self._tptr(hs), C.c_void_p(self._stream())))
+        return lr[:got], hs[:got]
+
     # ---- resident (benchmark) path -------------------------------------------------------------------------------
     def resident_load(self, dev: int, raw: np.ndarray) -> None:
         raw = np.ascontiguousarray(raw)
@@ -242,6 +340,7 @@ class Engine:
     # ---- mixers ---------------------------------------------------------------------------------------------------
     def configure_mixers(self, mixers: Sequence[Sequence[Tuple[int, int, float, float]]]) -> None:
         """mixers[m] = [(dev, chan, ampfactor, balance), ...]"""
+        self._n_mixers = len(mixers)
         offs = [0]
         flat = []
         for m in mixers:
